@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — learner gradient-steps/sec (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one `learn()` call of the hot path (`ReplayBuffer.sample ->
 PolicyLearner.learn()`) with `training_rounds = --rounds` gradient steps at
@@ -22,6 +22,8 @@ than the 126 MB L2, so sampled rows come from HBM.
                   host cores, the reference's own algorithm) on a bounded sample
 `--impl reference` times that CPU port alone (rank 0), same metric/config.
 N > 1: one process per GPU, each with its own buffer shard (see DESIGN.md §multi-GPU).
+`--dump-outputs DIR` writes what the last timed call computed (rank 0) as .npy files in DIR; the
+inputs are seeded, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -293,11 +295,13 @@ def run_b200(args) -> None:
     kernel_ms = []
     e0.record()
     for _ in range(args.steps):
-        group.learn()
+        reports = group.learn()
         kernel_ms.append(group.last_kernel_ms())
     e1.record()
     barrier()
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, reports, learners)
     t = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -326,7 +330,7 @@ def run_b200(args) -> None:
         e2e_step()
     barrier()
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e2e_steps = max(3, args.steps // 2)
+    e2e_steps = args.steps
     f0.record()
     for _ in range(e2e_steps):
         last_loss = e2e_step()
@@ -446,6 +450,25 @@ def run_b200(args) -> None:
         dist.destroy_process_group()
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, reports: list, learners: list) -> None:
+    """What the caller of the last timed group.learn() receives, as float32 .npy files: loss.npy [k, rounds] (the
+    reports) and parameters.npy / target_parameters.npy [k, P] (the online and target networks that call left).
+    k is every learner unless that exceeds DUMP_BYTES; then it is the first k, which are the same learners
+    with the same buffers and seeds whatever the learner count."""
+    import numpy as np
+    import torch
+    rounds, p = len(reports[0]["loss"]), learners[0].flat_parameters.numel()
+    k = max(1, min(len(learners), DUMP_BYTES // (4 * (rounds + 2 * p))))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "loss.npy"), np.asarray([r["loss"] for r in reports[:k]], dtype=np.float32))
+    np.save(os.path.join(path, "parameters.npy"), torch.stack([l.flat_parameters for l in learners[:k]]).float().cpu().numpy())
+    np.save(os.path.join(path, "target_parameters.npy"),
+            torch.stack([l.flat_target_parameters for l in learners[:k]]).float().cpu().numpy())
+
+
 def dp_record(args, dev, rank, world, make_learner, barrier) -> dict:
     """ONE DeepQLearning learner at world = N (SURVEY.md 8e): the 1e6-transition replay buffer is sharded by interleaved
     global write counter (rank g mod W), every rank runs the SAME MT19937 stream and so draws the same 256 global indices
@@ -527,13 +550,13 @@ def dp_record(args, dev, rank, world, make_learner, barrier) -> dict:
         parity["verdict"] = "ok" if ok else "FAILED"
     # ---- timing
     dp._training_rounds = rounds
-    sec, upd = clocked(dp, shard, max(3, args.steps // 4))
+    sec, upd = clocked(dp, shard, args.steps)
     t = torch.tensor([sec], device=dev)
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
     out = None
     if rank == 0:
         solo._training_rounds = rounds
-        ssec, supd = clocked_solo(solo, full, max(3, args.steps // 4), rounds, dev)
+        ssec, supd = clocked_solo(solo, full, args.steps, rounds, dev)
         out = {"what": f"ONE DeepQLearning learner, replay of {cap} transitions sharded over {world} GPUs (interleaved ownership), the same "
                        f"{BATCH} global indices per round on every rank, in-kernel NVLink exchange of the partial gradient (+ sum |q - y|)",
                "value": rounds / float(t.item()), "unit": "gradient-steps/s (one sequential learner)", "world": world,
@@ -810,7 +833,11 @@ def main() -> None:
     ap.add_argument("--dp-rounds", type=int, default=256)
     ap.add_argument("--no-extras", action="store_true", help="skip the SAC / PPO / prioritized-replay side measurements")
     ap.add_argument("--extras-only", action="store_true", help="developer: run only the side measurements on cuda:0")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the losses and parameters of the last timed step to DIR/*.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries the ONE JSON line and nothing else: libraries that print there (NCCL's version banner, torch warnings
     # routed to fd 1) are sent to stderr for the duration of the run; print() is bound to the saved descriptor
     global print

@@ -1,7 +1,7 @@
 """CPU-side checks: the C-ABI library loads and exports every symbol the header
 declares (no compute without a GPU), the product fails loudly without CUDA, host
-logic (layout arithmetic, error mapping), and — when the reference is present in
-this container — that the plugins subclass Pearl's own base classes."""
+logic (layout arithmetic, error mapping), and — where facebookresearch/Pearl is
+available (tests/_pearl.py) — that the plugins subclass Pearl's own base classes."""
 import ctypes
 import os
 import re
@@ -10,6 +10,7 @@ import sys
 
 import pytest
 
+from _pearl import PEARL_ROOT
 from conftest import ROOT
 
 HEADER = os.path.join(ROOT, "include", "pearl_b200.h")
@@ -87,10 +88,10 @@ def test_product_never_imports_the_oracle():
                 assert not bad.search(src), f"{f} uses the oracle"
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/pearl"), reason="reference not present (GPU box)")
+@pytest.mark.skipif(PEARL_ROOT is None, reason="facebookresearch/Pearl is not available")
 def test_plugins_subclass_pearl_when_available():
     code = (
-        "import sys; sys.path[:0]=[%r, '/root/reference', %r]\n"
+        "import sys; sys.path[:0]=[%r, %r, %r]\n"
         "import pearl_b200\n"
         "from pearl.replay_buffers.replay_buffer import ReplayBuffer\n"
         "from pearl.policy_learners.sequential_decision_making.deep_q_learning import DeepQLearning\n"
@@ -120,19 +121,19 @@ def test_plugins_subclass_pearl_when_available():
         "    assert 'no CPU path' in str(e)\n"
         "from pearl.replay_buffers.transition import TransitionBatch\n"
         "assert pearl_b200.TransitionBatch is TransitionBatch\n"
-        "print('ok')\n" % (os.path.join(ROOT, "oracle", "stubs"), ROOT))
+        "print('ok')\n" % (os.path.join(ROOT, "oracle", "stubs"), PEARL_ROOT, ROOT))
     env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env)
     assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-2000:]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/pearl"), reason="reference not present (GPU box)")
+@pytest.mark.skipif(PEARL_ROOT is None, reason="facebookresearch/Pearl is not available")
 def test_actor_critic_plugins_bind_reference_modules_to_flat_vectors():
     """Host logic of pearl_b200/actor_critic.py against a stand-in learner (tests/actor_critic_host_worker.py): constructor
     arguments, parameters / AdamW state as views, step counts, SAC's entropy block, checkpoint import into a fresh and into an
     already bound learner, refusal of unsupported optimizers and network shapes."""
     env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "actor_critic_host_worker.py"), "/root/reference"],
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "actor_critic_host_worker.py"), PEARL_ROOT],
                          capture_output=True, text=True, env=env, timeout=600)
     assert out.returncode == 0 and "ACTOR_CRITIC_HOST_OK" in out.stdout, (out.stdout[-1500:], out.stderr[-4000:])
 

@@ -1,20 +1,17 @@
 """PearlAgent (the reference's own facade, pearl/pearl_agent.py) on top of the CUDA path.  Needs facebookresearch/Pearl
-importable: its root is taken from $PEARL_REFERENCE_ROOT, /root/reference, or a scratch copy under oracle/_ref/ (git-ignored;
-staged only for validation runs on the GPU box, see profiles/r2_pearl_agent_gpu.md).  Skipped otherwise."""
+(tests/_pearl.py: the build of it in oracle/_ref/, $PEARL_REFERENCE_ROOT or an importable `pearl`).  Skipped otherwise."""
 import os
 import subprocess
 import sys
 
 import pytest
 
+from _pearl import PEARL_ROOT as REF
 from conftest import ROOT
-
-CANDIDATES = [os.environ.get("PEARL_REFERENCE_ROOT", ""), "/root/reference", os.path.join(ROOT, "oracle", "_ref", "reference")]
-REF = next((c for c in CANDIDATES if c and os.path.isdir(os.path.join(c, "pearl"))), None)
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(REF is None, reason="facebookresearch/Pearl is not available on this box")
+@pytest.mark.skipif(REF is None, reason="facebookresearch/Pearl is not available")
 def test_pearl_agent_drives_the_b200_plugins_like_the_reference_plugins():
     env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "pearl_agent_worker.py"), REF], capture_output=True, text=True,
@@ -24,7 +21,7 @@ def test_pearl_agent_drives_the_b200_plugins_like_the_reference_plugins():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(REF is None, reason="facebookresearch/Pearl is not available on this box")
+@pytest.mark.skipif(REF is None, reason="facebookresearch/Pearl is not available")
 def test_actor_critic_plugins_subclass_the_reference_and_run_under_pearl_agent():
     """SAC / TD3 / DDPG / PPO: the plugins are the reference classes with learn() replaced (pearl_b200/actor_critic.py)."""
     env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")

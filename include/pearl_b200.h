@@ -372,6 +372,50 @@ int prl_sac_learn(prl_sac *sac, prl_buf *buf, int rounds, int batch, const float
 int prl_sac_set_graph(prl_sac *sac, int enable);
 int64_t prl_sac_last_launches(const prl_sac *sac);
 
+/* ---- discrete Soft Actor-Critic -----------------------------------------------------------------
+ * Replaces SoftActorCritic.learn_batch (policy_learners/sequential_decision_making/soft_actor_critic.py:151-286 on
+ * actor_critic_base.py:309-366) driven by PolicyLearner.learn (policy_learner.py:162-204) over a discrete-action ring with a
+ * fixed action space: per round sample -> actor step (p = softmax(actor(s)), loss = mean over B x A of
+ * p (alpha log(p + 1e-8) - min(Q1, Q2)(s, .)), :247-286) -> critic step with the updated actor (y = r + gamma (1 - terminated)
+ * sum_a p'(min(Q1t, Q2t)(s', a) - alpha log(p' + 1e-8)), twin MSE, :180-245, critic_utils.py:170-203) -> soft target update
+ * (tau every round, critic_utils.py:103-122) -> [autotune] entropy step: loss = exp(log_alpha) (H - target_entropy),
+ * H = -mean_b sum_a p log(p + 1e-8) of the actor step's p, torch.optim.Adam(eps = entropy_eps) (:137-142, 151-178).
+ * Actor and critics: AdamW(amsgrad), one step count.  The step draws no random numbers.
+ * Flat parameter layouts (fp32, row-major [out][in] like nn.Linear):
+ *   actor : W1[h1][obs] b1 W2[h2][h1] b2 W3[A][h2] b3
+ *   critic: TWO consecutive copies (q1 then q2) of W1[c1][obs+A] b1 W2[c2][c1] b2 W3[1][c2] b3   (input = state || one_hot(a)) */
+typedef struct prl_dsac_cfg {
+    int32_t obs_dim, n_actions, actor_h1, actor_h2, critic_h1, critic_h2;
+    int32_t autotune;     /* entropy_autotune */
+    int32_t max_batch, max_rounds;
+    double actor_lr, critic_lr, entropy_lr, beta1, beta2, eps, weight_decay, gamma, tau;
+    double target_entropy; /* -target_entropy_scale * log(1 / n_actions), as the reference evaluates it in fp32 */
+    double entropy_eps;    /* eps of the entropy optimizer (the reference: 1e-4) */
+} prl_dsac_cfg;
+typedef struct prl_dsac prl_dsac;
+int64_t prl_dsac_actor_param_count(const prl_dsac_cfg *cfg);
+int64_t prl_dsac_critic_param_count(const prl_dsac_cfg *cfg);   /* ONE critic */
+int64_t prl_dsac_workspace_bytes(const prl_dsac_cfg *cfg);
+/* All pointers are device memory owned by the caller: actor vectors f32[actor_param_count], critic vectors
+ * f32[2 * critic_param_count], log_alpha4 = {log_alpha, Adam exp_avg, Adam exp_avg_sq, unused}, alpha1 = the entropy
+ * coefficient in use (fixed when autotune = 0).  adam_step: optimizer steps already taken (all three optimizers). */
+int prl_dsac_create(prl_dsac **out, const prl_dsac_cfg *cfg, float *actor_w, float *actor_m, float *actor_v,
+                    float *actor_vmax, float *critic_w, float *critic_m, float *critic_v, float *critic_vmax,
+                    float *critic_target_w, float *log_alpha4, float *alpha1, int64_t adam_step, void *workspace);
+int prl_dsac_destroy(prl_dsac *dsac);
+int64_t prl_dsac_adam_step(const prl_dsac *dsac);
+/* New actor / critic learning rates, used from the next prl_dsac_learn on (the per-round optimizer scalars are computed
+ * at every call, so a captured round is kept): SoftActorCritic.reset steps an ExponentialLR of the actor every episode. */
+int prl_dsac_set_lr(prl_dsac *dsac, double actor_lr, double critic_lr);
+/* out_*_loss: device f32[rounds] (out_entropy_loss: the entropy loss of autotune rounds, untouched otherwise);
+ * out_logical_dev (optional) i32[rounds][batch] = sampled indices.  PRL_EINVAL without device work for a continuous-action
+ * buffer, a buffer with PRL_BUF_DYNAMIC_ACTIONS, a sharded buffer or mismatched dimensions. */
+int prl_dsac_learn(prl_dsac *dsac, prl_buf *buf, int rounds, int batch, float *out_actor_loss_dev, float *out_critic_loss_dev,
+                   float *out_entropy_loss_dev, int32_t *out_logical_dev, void *stream);
+/* CUDA-graph replay of the round (default on; 0 = plain stream launches).  Kernels launched by the last learn. */
+int prl_dsac_set_graph(prl_dsac *dsac, int enable);
+int64_t prl_dsac_last_launches(const prl_dsac *dsac);
+
 /* ---- TD3 / DDPG ----------------------------------------------------------------------------------
  * Replaces TD3.learn_batch (policy_learners/sequential_decision_making/td3.py:106-202) and, with
  * actor_update_freq = 1 and no noise, DeepDeterministicPolicyGradient (ddpg.py:105-157 on

@@ -12,12 +12,13 @@ from .replay_buffer import B200ReplayBuffer  # noqa: F401
 from .per import B200PrioritizedReplayBuffer  # noqa: F401
 from .her import B200HindsightExperienceReplayBuffer  # noqa: F401
 from .ppo import gae_and_lambda_returns  # noqa: F401
-# subclasses of the reference's ContinuousSoftActorCritic / ProximalPolicyOptimization / TD3 / DDPG when Pearl is importable,
+# subclasses of the reference's ContinuousSoftActorCritic / SoftActorCritic / ProximalPolicyOptimization / TD3 / DDPG when Pearl
+# is importable,
 # the stand-alone CUDA learners (same keyword arguments) otherwise
 from .actor_critic import (B200ContinuousSoftActorCritic, B200DeepDeterministicPolicyGradient,  # noqa: F401
-                           B200ProximalPolicyOptimization, B200TD3)
+                           B200ProximalPolicyOptimization, B200SoftActorCritic, B200TD3)
 from .dist import B200Communicator, all_gather_bytes, shard_owner  # noqa: F401
 
 __all__ = ["B200ReplayBuffer", "B200DeepQLearning", "B200DoubleDQN", "TransitionBatch",
-           "OneHotActionTensorRepresentationModule", "HAVE_PEARL", "B200Communicator", "B200LearnerGroup", "B200PrioritizedReplayBuffer", "gae_and_lambda_returns", "B200ContinuousSoftActorCritic", "B200ProximalPolicyOptimization",
+           "OneHotActionTensorRepresentationModule", "HAVE_PEARL", "B200Communicator", "B200LearnerGroup", "B200PrioritizedReplayBuffer", "gae_and_lambda_returns", "B200ContinuousSoftActorCritic", "B200SoftActorCritic", "B200ProximalPolicyOptimization",
            "B200TD3", "B200DeepDeterministicPolicyGradient", "B200HindsightExperienceReplayBuffer"]

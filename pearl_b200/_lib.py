@@ -41,6 +41,14 @@ class SacCfg(C.Structure):
                 ("tau", C.c_double)]
 
 
+class DsacCfg(C.Structure):
+    _fields_ = [("obs_dim", C.c_int32), ("n_actions", C.c_int32), ("actor_h1", C.c_int32), ("actor_h2", C.c_int32),
+                ("critic_h1", C.c_int32), ("critic_h2", C.c_int32), ("autotune", C.c_int32), ("max_batch", C.c_int32),
+                ("max_rounds", C.c_int32), ("actor_lr", C.c_double), ("critic_lr", C.c_double), ("entropy_lr", C.c_double),
+                ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double), ("weight_decay", C.c_double),
+                ("gamma", C.c_double), ("tau", C.c_double), ("target_entropy", C.c_double), ("entropy_eps", C.c_double)]
+
+
 class Td3Cfg(C.Structure):
     _fields_ = [("obs_dim", C.c_int32), ("act_dim", C.c_int32), ("actor_h1", C.c_int32), ("actor_h2", C.c_int32),
                 ("critic_h1", C.c_int32), ("critic_h2", C.c_int32), ("actor_update_freq", C.c_int32), ("max_batch", C.c_int32),
@@ -125,6 +133,16 @@ _SIGNATURES = {
     "prl_sac_set_graph": (C.c_int, [_P, C.c_int]),
     "prl_sac_last_launches": (C.c_int64, [_P]),
     "prl_sac_learn": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]),
+    "prl_dsac_actor_param_count": (C.c_int64, [C.POINTER(DsacCfg)]),
+    "prl_dsac_critic_param_count": (C.c_int64, [C.POINTER(DsacCfg)]),
+    "prl_dsac_workspace_bytes": (C.c_int64, [C.POINTER(DsacCfg)]),
+    "prl_dsac_create": (C.c_int, [C.POINTER(_P), C.POINTER(DsacCfg)] + [_P] * 11 + [C.c_int64, _P]),
+    "prl_dsac_destroy": (C.c_int, [_P]),
+    "prl_dsac_adam_step": (C.c_int64, [_P]),
+    "prl_dsac_set_lr": (C.c_int, [_P, C.c_double, C.c_double]),
+    "prl_dsac_learn": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P]),
+    "prl_dsac_set_graph": (C.c_int, [_P, C.c_int]),
+    "prl_dsac_last_launches": (C.c_int64, [_P]),
     "prl_td3_actor_param_count": (C.c_int64, [C.POINTER(Td3Cfg)]),
     "prl_td3_critic_param_count": (C.c_int64, [C.POINTER(Td3Cfg)]),
     "prl_td3_workspace_bytes": (C.c_int64, [C.POINTER(Td3Cfg)]),

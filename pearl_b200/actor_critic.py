@@ -1,6 +1,7 @@
 """Actor-critic plugins that SUBCLASS the reference classes (SURVEY.md §8 rows a1 / a14-a16, f3):
 
     B200ContinuousSoftActorCritic   (ContinuousSoftActorCritic, soft_actor_critic_continuous.py:42-231)
+    B200SoftActorCritic             (SoftActorCritic, soft_actor_critic.py:48-286; discrete actions)
     B200ProximalPolicyOptimization  (ProximalPolicyOptimization, ppo.py:96-293)
     B200TD3 / B200DeepDeterministicPolicyGradient  (td3.py:43-202, ddpg.py:41-157)
 
@@ -9,7 +10,7 @@ constructor runs unchanged (same arguments, same networks, same optimizers, same
 `pearl.pearl_agent.PearlAgent` accepts them as they are, `act()` / `reset()` / `compare()` / `state_dict()` are the
 reference's own code.  On the first `learn()` (after PearlAgent moved the learner to its CUDA device) the parameters of
 `_actor`, `_critic` (and their targets) are re-pointed at views into the flat fp32 vectors of the CUDA learner
-(`pearl_b200.sac / ppo / td3`), and `optimizer.state` at views into its flat AdamW vectors: the kernels and torch see the
+(`pearl_b200.sac / dsac / ppo / td3`), and `optimizer.state` at views into its flat AdamW vectors: the kernels and torch see the
 same memory, nothing is copied per call, `get_extra_state` / `set_extra_state` (actor_critic_base.py:411-428) checkpoint
 the live state, and a state loaded with `load_state_dict` is picked up on the next `learn()`.
 
@@ -22,6 +23,7 @@ from typing import Any
 
 import torch
 
+from .dsac import B200SoftActorCritic as DsacCore
 from .ppo import B200ProximalPolicyOptimization as PpoCore
 from .sac import B200ContinuousSoftActorCritic as SacCore
 from .td3 import B200DeepDeterministicPolicyGradient as DdpgCore
@@ -30,6 +32,7 @@ from .td3 import B200TD3 as Td3Core
 try:  # pragma: no cover - depends on the environment
     from pearl.policy_learners.sequential_decision_making.ddpg import DeepDeterministicPolicyGradient as _RefDDPG
     from pearl.policy_learners.sequential_decision_making.ppo import ProximalPolicyOptimization as _RefPPO
+    from pearl.policy_learners.sequential_decision_making.soft_actor_critic import SoftActorCritic as _RefDSAC
     from pearl.policy_learners.sequential_decision_making.soft_actor_critic_continuous import (
         ContinuousSoftActorCritic as _RefSAC,
     )
@@ -265,6 +268,104 @@ if HAVE_REFERENCE:
             if self._entropy_autotune:
                 _set_steps(self._entropy_optimizer, self._core_steps(core)[0])
 
+    def _entropy_adam_lr(opt: torch.optim.Optimizer) -> float:
+        """The CUDA learner's entropy step is torch.optim.Adam(eps=1e-4) with default betas, no weight decay, no amsgrad
+        (what SoftActorCritic constructs, soft_actor_critic.py:126-133)."""
+        g = opt.param_groups[0] if type(opt) is torch.optim.Adam and len(opt.param_groups) == 1 else None
+        if (g is None or g.get("amsgrad", False) or g.get("maximize", False) or tuple(g["betas"]) != (0.9, 0.999)
+                or float(g["eps"]) != 1e-4 or float(g["weight_decay"]) != 0.0):
+            raise NotImplementedError("entropy optimizer: the CUDA learner implements torch.optim.Adam(eps=1e-4, betas=(0.9, 0.999), "
+                                      "weight_decay=0, amsgrad=False) in one parameter group")
+        return float(g["lr"])
+
+    class B200SoftActorCritic(_B200ActorCriticMixin, _RefDSAC):
+        """Drop-in for `pearl...soft_actor_critic.SoftActorCritic` (discrete actions, fixed action space).  `reset()` steps the
+        reference's ExponentialLR of the actor every episode; the new rate reaches the CUDA learner through prl_dsac_set_lr
+        without re-creating its handle or re-capturing its round."""
+
+        def _make_core(self, device):
+            from pearl.action_representation_modules.one_hot_action_representation_module import (
+                OneHotActionTensorRepresentationModule,
+            )
+            from pearl.neural_networks.sequential_decision_making.actor_networks import VanillaActorNetwork
+            from pearl.neural_networks.sequential_decision_making.q_value_networks import VanillaQValueNetwork
+            from pearl.neural_networks.sequential_decision_making.twin_critic import TwinCritic
+            critic = self._critic
+            if (type(self._actor) is not VanillaActorNetwork or not isinstance(critic, TwinCritic)
+                    or not all(type(c) is VanillaQValueNetwork for c in (critic._critic_1, critic._critic_2))):
+                raise NotImplementedError("the CUDA discrete SAC learner is built for VanillaActorNetwork + TwinCritic(VanillaQValueNetwork)")
+            sa, sc = _shapes(self._actor), _shapes(critic)
+            if len(sa) != 6 or len(sc) != 12:
+                raise NotImplementedError("the CUDA discrete SAC learner is built for two hidden layers in the actor and in each critic")
+            obs, h1, h2, n_act = _mlp3(sa, "actor")
+            dq, c1, c2, one = _mlp3(sc[:6], "critic")
+            arm = self.action_representation_module
+            if (not isinstance(arm, OneHotActionTensorRepresentationModule) or int(arm.max_number_actions) != n_act
+                    or dq != obs + n_act or one != 1 or sc[6:] != sc[:6]):
+                raise NotImplementedError("the CUDA discrete SAC learner needs a one-hot action representation of the actor's "
+                                          "n_actions and critics over state || one-hot action")
+            hsm = getattr(self, "_history_summarization_module", None)
+            if hsm is not None and any(True for _ in hsm.parameters()):
+                raise NotImplementedError("the CUDA discrete SAC learner takes states as they are: a history summarization "
+                                          "module with parameters (e.g. LSTM) is not supported")
+            core = DsacCore(state_dim=obs, n_actions=n_act, actor_hidden_dims=[h1, h2], critic_hidden_dims=[c1, c2],
+                            actor_learning_rate=_adamw_lr(self._actor_optimizer, "actor optimizer"),
+                            critic_learning_rate=_adamw_lr(self._critic_optimizer, "critic optimizer"),
+                            critic_soft_update_tau=float(self._critic_soft_update_tau), discount_factor=float(self._discount_factor),
+                            training_rounds=int(self._training_rounds), batch_size=int(self._batch_size),
+                            entropy_coef=float(self._entropy_coef), entropy_autotune=bool(self._entropy_autotune),
+                            device=device, **self._b200_opts)
+            if self._entropy_autotune:
+                core._target_entropy = float(self._target_entropy)
+                core._entropy_learning_rate = _entropy_adam_lr(self._entropy_optimizer)
+            return core
+
+        def _module_pairs(self, core):
+            return [(self._actor, core.actor_params), (self._critic, core.critic_params), (self._critic_target, core.critic_target_params)]
+
+        def _core_steps(self, core):
+            s = core.adam_step()
+            return (s, s)
+
+        def _restart_core(self, core, steps):
+            if steps[0] != steps[1]:
+                raise NotImplementedError("discrete SAC steps its actor and critics once per round: one AdamW step count")
+            if core._handle.value and tuple(steps) == self._core_steps(core):
+                # only the learning rates changed (ExponentialLR at every reset()): keep the handle and its captured round
+                core.set_learning_rates(core._actor_learning_rate, core._critic_learning_rate)
+                return
+            core._release()
+            core._adam_step = int(steps[0])
+
+        def _bind_extras(self, core):
+            """Entropy coefficient: `_log_entropy` (Parameter) and its Adam state are views of the CUDA learner's log-entropy
+            block, `_entropy_coef` (buffer, shape kept) a view of its coefficient.  A state loaded into the entropy optimizer
+            since the last call is imported."""
+            coef = core._entropy_coef
+            if self._entropy_coef.data_ptr() != coef.data_ptr():
+                coef.copy_(self._entropy_coef.detach().reshape(1).to(coef))
+                self._entropy_coef = coef.view(self._entropy_coef.shape)
+            if not self._entropy_autotune:
+                return
+            lr = _entropy_adam_lr(self._entropy_optimizer)
+            if lr != core._entropy_learning_rate:        # part of the handle's configuration
+                core._entropy_learning_rate = lr
+                core._release()
+            blk, p, st = core._log_entropy, self._log_entropy, self._entropy_optimizer.state
+            if p.data_ptr() != blk.data_ptr():
+                blk[0:1].copy_(p.detach().reshape(1).to(blk))
+                p.data = blk[0:1]
+            if p in st and "exp_avg" in st[p] and st[p]["exp_avg"].data_ptr() == blk[1:2].data_ptr():
+                return
+            if p in st and "exp_avg" in st[p]:
+                blk[1:2].copy_(st[p]["exp_avg"].reshape(1))
+                blk[2:3].copy_(st[p]["exp_avg_sq"].reshape(1))
+            st[p] = dict(step=torch.tensor(float(self._core_steps(core)[0])), exp_avg=blk[1:2], exp_avg_sq=blk[2:3])
+
+        def _after_learn(self, core):
+            if self._entropy_autotune:
+                _set_steps(self._entropy_optimizer, self._core_steps(core)[0])
+
     class B200ProximalPolicyOptimization(_B200ActorCriticMixin, _RefPPO):
         """Drop-in for `pearl...ppo.ProximalPolicyOptimization` (discrete actions, as the reference's `_actor_loss`)."""
 
@@ -357,6 +458,7 @@ if HAVE_REFERENCE:
 
 else:
     B200ContinuousSoftActorCritic = SacCore
+    B200SoftActorCritic = DsacCore
     B200ProximalPolicyOptimization = PpoCore
     B200TD3 = Td3Core
     B200DeepDeterministicPolicyGradient = DdpgCore

@@ -7,7 +7,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SRC = [os.path.join(HERE, "csrc", f) for f in ("replay_buffer.cu", "dqn.cu", "dqn_tc.cu", "ppo.cu", "per.cu", "sac.cu", "td3.cu", "gemm_tc.cu", "umma_test.cu")]
+SRC = [os.path.join(HERE, "csrc", f) for f in ("replay_buffer.cu", "dqn.cu", "dqn_tc.cu", "ppo.cu", "per.cu", "sac.cu", "dsac.cu", "td3.cu", "gemm_tc.cu", "umma_test.cu")]
 HDR = [os.path.join(HERE, "csrc", "common.cuh"), os.path.join(HERE, "csrc", "sampler.cuh"), os.path.join(HERE, "csrc", "umma.cuh"), os.path.join(HERE, "csrc", "dqn_common.cuh"), os.path.join(HERE, "csrc", "gemm.cuh"), os.path.join(os.path.dirname(HERE), "include", "pearl_b200.h")]
 OUT = os.path.join(HERE, "libpearlb200.so")
 

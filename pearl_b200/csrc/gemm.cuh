@@ -274,6 +274,24 @@ static __global__ void k_head_bwd(int B, int H, const float *__restrict__ dq, co
     dc2[o] = (c2[o] > 0.f) ? dq[z * B + m] * __ldg(w3 + z * w_net_stride + j) : 0.f;
 }
 
+// twin-critic MSE (critic_utils.py:170-203): loss = (mse(q1, y) + mse(q2, y)) / 2 with q = [2][B], and its gradient
+// dq_i = (q_i - y) / B.  Called by every thread of ONE block of 256 (fixed summation order); the loss is returned to thread 0.
+__device__ __forceinline__ float twin_mse_block(int B, const float *__restrict__ q, const float *__restrict__ y, float *__restrict__ dq) {
+    __shared__ float red[256];
+    float s = 0.f;
+    const float ib = 1.f / (float)B;
+    for (int b = threadIdx.x; b < B; b += blockDim.x) {
+        const float e1 = q[b] - y[b], e2 = q[B + b] - y[b];
+        s += e1 * e1 + e2 * e2;
+        dq[b] = e1 * ib;            // d/dq1 of (mse1 + mse2) / 2
+        dq[B + b] = e2 * ib;
+    }
+    red[threadIdx.x] = s;
+    __syncthreads();
+    for (int o = 128; o; o >>= 1) { if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o]; __syncthreads(); }
+    return red[0] * ib * 0.5f;
+}
+
 struct AdamHp { float decay, omb1, beta2, omb2, eps; };
 __device__ __forceinline__ float adamw1(float w, float &m, float &v, float &x, float g, const AdamHp &h, float step_size, float bc2s) {
     float p = __fmul_rn(w, h.decay);

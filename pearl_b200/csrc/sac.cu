@@ -125,19 +125,8 @@ __global__ void k_sac_target(int B, const float *__restrict__ qt, const float *_
 }
 __global__ void k_sac_critic_loss(int B, const float *__restrict__ q, const float *__restrict__ y, float *__restrict__ dq,
                                   const SacCall *__restrict__ call, const int *__restrict__ round_idx) {
-    __shared__ float red[256];
-    float s = 0.f;
-    const float ib = 1.f / (float)B;
-    for (int b = threadIdx.x; b < B; b += blockDim.x) {
-        const float e1 = q[b] - y[b], e2 = q[B + b] - y[b];
-        s += e1 * e1 + e2 * e2;
-        dq[b] = e1 * ib;            // d/dq1 of (mse1 + mse2) / 2
-        dq[B + b] = e2 * ib;
-    }
-    red[threadIdx.x] = s;
-    __syncthreads();
-    for (int o = 128; o; o >>= 1) { if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o]; __syncthreads(); }
-    if (threadIdx.x == 0) call->out_critic[*round_idx] = red[0] * ib * 0.5f;
+    const float loss = twin_mse_block(B, q, y, dq);
+    if (threadIdx.x == 0) call->out_critic[*round_idx] = loss;
 }
 
 // entropy coefficient: loss = mean(-exp(log_alpha) * (logp + target_entropy)); AdamW on the scalar; alpha = exp(log_alpha)
